@@ -7,7 +7,7 @@ One "step" = one full pass of the hot path over the resident synthetic lineitem 
   stage 3  ShuffleReader -> SortPreservingMergeExec -> ShuffleWriter(None)
 exactly the stage shapes Ballista's planner emits for q1 (ballista/scheduler/src/planner.rs:655-670).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 N>1 is launched by the driver under torchrun (one rank per GPU, NCCL); every rank owns SF10 worth
 of lineitem rows (weak scaling: the global table is SF(10*N)), the partial aggregate states are
 exchanged with an NCCL all-to-all, and `value` is global rows / max-over-ranks device time.
@@ -204,8 +204,7 @@ def cpu_q1(msf: int, row_begin: int, row_end: int, threads: int, steps: int, war
     import oracle_ffi
     from concurrent.futures import ThreadPoolExecutor
     from ballista_b200 import tpch
-    oracle_ffi.build()
-    eng = oracle_ffi.OracleEngine()
+    eng = oracle_ffi.OracleEngine()     # loads the oracle/liboracle.so the build made: no `make` in a tree that may be read-only
     parts = threads
     rows = row_end - row_begin
     step = (rows + parts - 1) // parts
@@ -248,7 +247,9 @@ def run_reference(args):
         emit({"impl": "reference", "unavailable": f"CPU arm implemented for the q1 headline workload only (asked: {args.workload})"})
         return
     rows = ROWS_SF10  # the FULL configs[1] table, like the GPU arm's per-GPU share
-    times, _ = cpu_q1(SF10_MSF, 0, rows, threads, args.steps, args.warmup)
+    times, res = cpu_q1(SF10_MSF, 0, rows, threads, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"q1": res})
     total = sum(times)
     value = rows * len(times) / total
     line = {
@@ -416,6 +417,8 @@ def run_b200(args):
 
     total_rows = ROWS_SF10 * world
     value = total_rows * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"q1": res})
 
     if trace:
         print(f"[trace rank {rank}] per-step ms: " + ", ".join(f"{k}={v / args.steps:.3f}" for k, v in tr.items()), file=sys.stderr)
@@ -543,7 +546,6 @@ def run_workload(args):
             eng.remove_job_data(f"par-{nme}")
         if rank == 0:
             import oracle_ffi
-            oracle_ffi.build()
             o = oracle_ffi.OracleEngine()
             for t, cols in tabs.items():
                 n = eng.tpch_table_rows(t, pmsf)
@@ -612,6 +614,8 @@ def run_workload(args):
     clocks = sampler.stop() if rank == 0 else None
     launches = eng.kernel_launches() - launches0
     kstats = eng.kernel_stats(reset=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
     # self-consistency at full scale (the oracle cannot hold SF100): a different shuffle fan-out must give the same table
     consistent = None
     if not args.no_parity:
@@ -723,6 +727,54 @@ def measure_e2e(eng, bb, pa, torch, dist, step, rank, world, device, steps):
                     "Decimal128 sign-extension bytes, H2D of h2d_bytes_per_step, device widens) -> 3 stages (+ exchanges) -> b200_partition_export (D2H)"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _column_to_numpy(col):
+    """One result column as float64 (nulls NaN); a string column as a float32 [rows, longest] matrix of its UTF-8 bytes,
+    zero-padded, a null row all NaN."""
+    import numpy as np
+    import pyarrow as pa
+    t = col.type
+    if pa.types.is_string(t) or pa.types.is_large_string(t) or pa.types.is_binary(t):
+        vals = [None if v is None else (v.encode() if isinstance(v, str) else v) for v in col.to_pylist()]
+        out = np.zeros((len(vals), max([1] + [len(v) for v in vals if v is not None])), np.float32)
+        for i, v in enumerate(vals):
+            if v is None:
+                out[i] = np.nan
+            else:
+                out[i, :len(v)] = np.frombuffer(v, np.uint8)
+        return out
+    if pa.types.is_date32(t):
+        col = col.cast(pa.int32())
+    elif pa.types.is_temporal(t):
+        col = col.cast(pa.int64())
+    return col.cast(pa.float64()).to_numpy(zero_copy_only=False).astype(np.float64)
+
+
+def dump_outputs(out_dir, results):
+    """results: {query: result table (pyarrow Table or RecordBatch) of the last timed step}.  Writes every column as
+    out_dir/<query>_<column>.npy.  Past DUMP_LIMIT_BYTES in all, each table keeps the same seeded sample of its rows
+    (in order) and its row numbers go to <query>__rows.npy."""
+    import numpy as np
+    import pyarrow as pa
+    os.makedirs(out_dir, exist_ok=True)
+    tables = {q: pa.Table.from_batches([r]) if isinstance(r, pa.RecordBatch) else r for q, r in results.items() if r is not None}
+    arrays = {q: [(name, _column_to_numpy(t.column(name))) for name in t.column_names] for q, t in tables.items()}
+    per_table = (DUMP_LIMIT_BYTES - (1 << 20)) // max(1, len(arrays))     # 1 MB left for the .npy headers
+    for q, cols in arrays.items():
+        n = tables[q].num_rows
+        row_bytes = sum(a.nbytes // max(1, n) for _, a in cols)
+        keep = n if row_bytes * n <= per_table else per_table // (row_bytes + 8)
+        if keep < n:
+            rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+            np.save(os.path.join(out_dir, f"{q}__rows.npy"), rows.astype(np.float64))
+            cols = [(name, a[rows]) for name, a in cols]
+        for name, a in cols:
+            np.save(os.path.join(out_dir, f"{q}_{name}.npy"), a)
+    log(f"dumped {sum(len(c) for c in arrays.values())} result columns of {sorted(arrays)} to {out_dir}")
+
+
 _REAL_STDOUT = None
 
 
@@ -754,7 +806,11 @@ def main():
     ap.add_argument("--no-fused-shuffle", action="store_true", help="N>1: always shuffle in two steps (writer, then NCCL exchange)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the result of the last one as DIR/<query>_<column>.npy "
+                                                          "(float64; strings as float32 byte matrices; at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -5,9 +5,10 @@ Fixtures: tests/golden/proto_plans.json -- every stage of the 22 TPC-H queries p
 datafusion.PhysicalPlanNode by google.protobuf with message classes built from the REFERENCE's .proto files
 (tests/golden/make_proto_plans.py; ballista/core/proto/*.proto).  Check: the typed plan (b200_plan_typed_json: resolved
 column indices, expression / aggregate types, every node's output schema) of the decoded IR equals the typed plan of the IR the
-bytes were generated from; both decoders of the fixture (this one and google.protobuf) must also agree on the proto itself
-when the reference's proto files are present."""
+bytes were generated from; the fixture bytes must also be, field for field, what google.protobuf read in them with the
+reference's message definitions (tests/golden/proto_plans_wire.json.gz)."""
 import base64
+import gzip
 import json
 import os
 
@@ -71,26 +72,66 @@ def test_malformed_and_unsupported_inputs():
     assert engine.plan_proto_to_json(proto + bytes([0x98, 0x06, 0x2a])) == engine.plan_proto_to_json(proto)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/ballista/core/proto/datafusion.proto"), reason="needs the reference's .proto files")
+def _read_varint(buf, i):
+    v = shift = 0
+    while True:
+        b = buf[i]
+        i += 1
+        v |= (b & 0x7f) << shift
+        shift += 7
+        if not b & 0x80:
+            return v, i
+
+
+def wire_fields(buf):
+    """[(field number, wire type, value)] of one protobuf message, schema-less: varints and fixed-width values as unsigned
+    ints, length-delimited values as bytes."""
+    out, i = [], 0
+    while i < len(buf):
+        key, i = _read_varint(buf, i)
+        num, wt = key >> 3, key & 7
+        if wt == 0:
+            v, i = _read_varint(buf, i)
+        elif wt in (1, 5):
+            n = 8 if wt == 1 else 4
+            v, i = int.from_bytes(buf[i:i + n], "little"), i + n
+        elif wt == 2:
+            n, i = _read_varint(buf, i)
+            v, i = bytes(buf[i:i + n]), i + n
+        else:
+            raise ValueError(f"wire type {wt}")
+        out.append((num, wt, v))
+    assert i == len(buf)
+    return out
+
+
+def _matches_tree(buf, tree):
+    fields = wire_fields(buf)
+    assert [(n, wt) for n, wt, _ in fields] == [(t[0], t[2]) for t in tree]
+    for (_, wt, v), (_, _, _, want) in zip(fields, tree):
+        if isinstance(want, list):
+            _matches_tree(v, want)
+        elif wt == 2:
+            assert base64.b64encode(v).decode() == want
+        else:
+            assert v == want
+
+
 def test_fixture_is_what_the_reference_protos_describe():
-    """google.protobuf, given the reference's message definitions, parses every fixture completely (no unknown fields), and a
-    re-serialisation is byte-identical: the fixtures are well-formed datafusion.PhysicalPlanNode messages."""
-    import sys
-    sys.path.insert(0, os.path.join(HERE, "golden"))
-    import protoc_lite
-    cls, _ = protoc_lite.load_ballista()
-    P = cls["datafusion.PhysicalPlanNode"]
-    B = cls["ballista.protobuf.BallistaPhysicalPlanNode"]
+    """Every fixture is, field for field, the datafusion.PhysicalPlanNode google.protobuf parsed from it with the reference's
+    message definitions (tests/golden/proto_plans_wire.json.gz, made by tests/golden/make_proto_wire.py, which also checked that
+    each parse had no unknown field and re-serialised byte-identically)."""
+    with gzip.open(os.path.join(HERE, "golden", "proto_plans_wire.json.gz"), "rt") as fh:
+        wire = json.load(fh)["cases"]
+    assert sorted(wire) == sorted(c["name"] for c in CASES)
     for c in CASES:
-        raw = base64.b64decode(c["proto_b64"])
-        m = P()
-        m.ParseFromString(raw)
-        assert m.SerializeToString() == raw
-        assert m.WhichOneof("PhysicalPlanType") == "extension"       # every stage is rooted at a Ballista shuffle writer
-        b = B()
-        b.ParseFromString(m.extension.node)
-        assert b.WhichOneof("PhysicalPlanType") in ("shuffle_writer", "sort_shuffle_writer")
-        assert len(m.extension.inputs) == 1
+        tree = wire[c["name"]]
+        _matches_tree(base64.b64decode(c["proto_b64"]), tree)
+        assert [f[1] for f in tree] == ["extension"]                  # every stage is rooted at a Ballista shuffle writer
+        ext = tree[0][3]
+        node = [f[3] for f in ext if f[1] == "node"]
+        assert len(node) == 1 and [f[1] for f in node[0]] in (["shuffle_writer"], ["sort_shuffle_writer"])
+        assert sum(f[1] == "inputs" for f in ext) == 1
 
 
 class _DecodedPlans:
