@@ -75,6 +75,7 @@ __global__ void agg_extract_kernel(AggTable T, AggExtractArgs A) {
   for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < T.cap; s += (unsigned long long)gridDim.x * blockDim.x) {
     if (T.state[s] != 2) continue;
     unsigned long long pos = atomicAdd(A.counter, 1ull);
+    if (pos >= A.cap) continue;
     for (int j = 0; j < A.n_out; j++) {
       const AggOut& o = A.out[j];
       switch (o.kind) {

@@ -47,6 +47,7 @@ struct AggExtractArgs {
   int n_out;
   int n_keys;
   unsigned long long* counter;   // device: rows emitted
+  unsigned long long cap;        // rows the outputs hold: groups past them are counted, not written
   unsigned int* error;           // device: RunStatus.error
 };
 void launch_agg_extract(const AggTable& T, const AggExtractArgs& A, cudaStream_t st);

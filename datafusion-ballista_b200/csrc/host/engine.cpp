@@ -84,6 +84,7 @@ struct b200_engine {
   uint64_t pf_bucket_slots = (uint64_t)1 << 19;  // partition-first aggregation: table slots per bucket (power of two; 0 = off)
   int64_t pf_min_rows = (int64_t)1 << 22;
   std::map<std::string, uint64_t> agg_groups;  // plan fingerprint -> most groups any task of that shape produced (sizes the table)
+  std::map<std::string, uint64_t> agg_spec;    // plan fingerprint + input partition -> groups of its last run, when the hinted sink held them at once
   void* pinned_stage = nullptr;              // small pinned buffer for status read-backs
   // ingest narrowing (import_batch): host pool + two pinned staging slots with their device mirrors
   std::unique_ptr<HostPool> pool;
@@ -118,13 +119,20 @@ struct b200_engine {
   std::mutex export_mu;                      // small-result export arena (pinned), one export at a time
   uint8_t* export_arena = nullptr;
   std::atomic<uint64_t> narrowed_bytes_saved{0};         // PCIe bytes not sent thanks to narrowing (b200_engine_counter)
+  std::atomic<uint64_t> stream_syncs{0};                 // host waits on the stream inside tasks and exports (b200_engine_counter)
+  // parsed stage plans, keyed by stage id + plan text (job id taken out when the caller names the job): the same stage of
+  // the next job is not parsed again.  The trees are shared read-only by every b200_stage prepared from them.
+  struct CachedPlan { std::shared_ptr<const PlanNode> plan; uint64_t used; };
+  std::map<std::string, CachedPlan> plan_cache;
+  uint64_t plan_cache_tick = 0;
 };
+static const size_t PLAN_CACHE_ENTRIES = 32;
 
 struct b200_stage {
   b200_engine* eng = nullptr;
   std::string job_id;
   int64_t stage_id = 0;
-  PlanPtr plan;
+  std::shared_ptr<const PlanNode> plan;  // shared with the engine's plan cache: read-only; its job_id is not this stage's
   std::string fingerprint;
   std::vector<OpMetrics> metrics;  // pre-order
   std::map<const PlanNode*, int> metric_index;
@@ -161,10 +169,15 @@ inline TaskCtx& task_ctx() {
   return t;
 }
 
+// Thrown by a deferred check when a task that ran on a remembered aggregate group count finds the count (or the sink) was
+// wrong: b200_stage_execute discards the task's outputs and runs it again without guessing.
+struct SpeculationMiss {};
+
 struct Exec {
   b200_engine* e;
   b200_stage* s;
   const volatile int32_t* cancel;
+  bool speculate = false;  // aggregates may run on the group count of their last run (run_aggregate); only b200_stage_execute retries
   cudaStream_t st() const { return e->stream; }
   void check_cancel() const {
     if (cancel && *cancel) throw EngineError(B200_ERR_CANCELLED, "task cancelled");
@@ -219,6 +232,7 @@ struct Exec {
   // wait for everything enqueued so far, then run the deferred checks (they may throw)
   void sync() const {
     TaskCtx& t = task_ctx();
+    e->stream_syncs++;
     cudaError_t se = cudaStreamSynchronize(st());
     t.drained = true;
     std::vector<std::function<void()>> cs;
@@ -226,6 +240,11 @@ struct Exec {
     CUDA_CHECK(se);
     for (auto& c : cs) c();
     check_cancel();
+  }
+  // wait for everything enqueued so far; deferred checks stay queued for the next sync()
+  void wait() const {
+    e->stream_syncs++;
+    CUDA_CHECK(cudaStreamSynchronize(st()));
   }
   // drop deferred checks without running them (error unwinding)
   static void abandon() {
@@ -819,23 +838,23 @@ std::vector<HostCol> download_batch(const Exec& x, const DevBatch& b, int64_t r0
         launch_bytes_to_bitmap(c.data, (uint8_t*)bm->ptr, n, nullptr, st);
         x.count();
         CUDA_CHECK(cudaMemcpyAsync(h.data.data(), bm->ptr, h.data.size(), cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
+        x.wait();
       }
     } else if (c.type.id == TypeId::Utf8) {
       DevColumn u = c.phys == PH_STRVIEW ? as_utf8(x, c) : c;
       h.data.resize((size_t)(n + 1) * 4);
       CUDA_CHECK(cudaMemcpyAsync(h.data.data(), u.data, h.data.size(), cudaMemcpyDeviceToHost, st));
-      CUDA_CHECK(cudaStreamSynchronize(st));
+      x.wait();
       int32_t* off = (int32_t*)h.data.data();
       int32_t first = off[0], last = off[n];
       h.extra.resize((size_t)(last - first));
       if (last > first) CUDA_CHECK(cudaMemcpyAsync(h.extra.data(), u.chars + first, h.extra.size(), cudaMemcpyDeviceToHost, st));
-      CUDA_CHECK(cudaStreamSynchronize(st));
+      x.wait();
       for (int64_t i = 0; i <= n; i++) off[i] -= first;
     } else {
       h.data.resize((size_t)n * c.width());
       if (n) CUDA_CHECK(cudaMemcpyAsync(h.data.data(), c.data, h.data.size(), cudaMemcpyDeviceToHost, st));
-      CUDA_CHECK(cudaStreamSynchronize(st));
+      x.wait();
     }
     hcs.push_back(std::move(h));
   }
@@ -853,6 +872,8 @@ void export_batch(const Exec& x, const DevBatch& b, int64_t r0, int64_t r1, Arro
 struct RunOutcome {
   RunStatus status;
   float ms = 0;
+  const RunStatus* deferred = nullptr;          // wait == false: the status word, readable after the task's next sync
+  const unsigned int* deferred_extra = nullptr;  // ... and the `extra_fetch` word
 };
 
 // the fused kernel's description of a program it can run instead of the tile VM (match_fused)
@@ -1052,6 +1073,8 @@ RunOutcome launch_program(const Exec& x, PipelineBuilder& pb, int reg_groups, co
       throw_run_error(hs->error);
     });
     memset(&o.status, 0, sizeof o.status);
+    o.deferred = hs;
+    o.deferred_extra = he;
     return o;
   }
   try {
@@ -1838,31 +1861,46 @@ struct TableMem {
 TableMem alloc_table(const Exec& x, uint64_t cap, int n_keys, const std::vector<AccDesc>& accs) {
   TableMem tm;
   memset(&tm.T, 0, sizeof tm.T);
-  auto A = [&](size_t bytes) {
-    DevPtr p = dev_alloc(bytes, x.st());
-    tm.keep.push_back(p);
-    return p->ptr;
-  };
+  // one allocation: [n_groups | hash | state | lock | acc] -- the part a fresh table needs initialised -- then the keys
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t nk = std::max<size_t>(1, (size_t)n_keys), na = std::max<size_t>(1, accs.size());
+  const size_t o_hash = 256, o_state = o_hash + up(cap * 8), o_lock = o_state + up(cap * 4), o_acc = o_lock + up(cap * 4);
+  const size_t o_keys = o_acc + up(na * cap * 16), o_kv = o_keys + up(nk * cap * 16), bytes = o_kv + up(nk * cap);
+  DevPtr blk = dev_alloc(bytes, x.st());
+  tm.keep.push_back(blk);
+  uint8_t* const b = (uint8_t*)blk->ptr;
   tm.T.cap = cap;
-  tm.T.hash = (unsigned long long*)A(cap * 8);
-  tm.T.state = (unsigned int*)A(cap * 4);
-  tm.T.lock = (unsigned int*)A(cap * 4);
-  tm.T.keys = (unsigned long long*)A(std::max<size_t>(1, (size_t)n_keys) * cap * 16);
-  tm.T.key_valid = (unsigned char*)A(std::max<size_t>(1, (size_t)n_keys) * cap);
-  tm.T.acc = (unsigned long long*)A(std::max<size_t>(1, accs.size()) * cap * 16);
-  tm.T.n_groups = (unsigned int*)A(16);
+  tm.T.n_groups = (unsigned int*)b;
+  tm.T.hash = (unsigned long long*)(b + o_hash);
+  tm.T.state = (unsigned int*)(b + o_state);
+  tm.T.lock = (unsigned int*)(b + o_lock);
+  tm.T.acc = (unsigned long long*)(b + o_acc);
+  tm.T.keys = (unsigned long long*)(b + o_keys);
+  tm.T.key_valid = (unsigned char*)(b + o_kv);
   AccKinds k;
   memset(&k, 0, sizeof k);
   k.n = (int)accs.size();
-  for (size_t i = 0; i < accs.size(); i++) k.kind[i] = accs[i].kind;
-  launch_agg_table_init(tm.T, k, x.st());
-  x.count();
+  bool zero_init = true;  // SUM / COUNT / AVG states start at 0; MIN / MAX start at the type's extreme
+  for (size_t i = 0; i < accs.size(); i++) {
+    k.kind[i] = accs[i].kind;
+    zero_init &= accs[i].kind != ACC_MIN_I128 && accs[i].kind != ACC_MAX_I128 && accs[i].kind != ACC_MIN_F64 && accs[i].kind != ACC_MAX_F64;
+  }
+  if (zero_init) {
+    CUDA_CHECK(cudaMemsetAsync(b, 0, o_keys, x.st()));
+  } else {
+    launch_agg_table_init(tm.T, k, x.st());
+    x.count();
+  }
   return tm;
 }
 
 typedef std::function<std::unique_ptr<PipelineBuilder>()> BuilderFactory;
 
-DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const PlanNode& node, const DevBatchPtr& src, OpMetrics* met) {
+// Largest aggregate output that a task may extract on the group count of its last run, before the count is read back
+// (the output block is zeroed so that rows the extraction does not write are empty values, never stray pointers).
+static const uint64_t SPEC_MAX_GROUPS = 4096;
+
+DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const PlanNode& node, const DevBatchPtr& src, OpMetrics* met, int part) {
   const int n_keys = (int)node.group_by.size();
   if (n_keys > VM_MAX_KEYS) throw EngineError(B200_ERR_UNSUPPORTED, "too many group-by columns");
   // initial optimism about the keys
@@ -1882,9 +1920,14 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
     if (it != x.s->metric_index.end()) node_idx = it->second;
   }
   const std::string hint_key = (x.s ? x.s->fingerprint : std::string("?")) + "#" + std::to_string(node_idx);
+  const std::string spec_key = hint_key + "@" + std::to_string(part);
   int level = 0;
   bool had_hint = false;
   uint64_t groups_hint = 0;
+  // a shape whose last run on this partition got its groups from the hinted sink at the first attempt: enqueue the extraction
+  // for that many groups without waiting; the status and the group count are checked at the task's final synchronisation
+  bool speculate = false;
+  uint64_t spec_groups = 0;
   {
     std::lock_guard<std::mutex> g(x.e->mu);
     auto it = x.e->agg_hint.find(hint_key);
@@ -1894,6 +1937,11 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
       had_hint = true;
       auto ig = x.e->agg_groups.find(hint_key);
       if (ig != x.e->agg_groups.end()) groups_hint = ig->second;
+      auto is = x.e->agg_spec.find(spec_key);
+      if (x.speculate && is != x.e->agg_spec.end()) {
+        speculate = true;
+        spec_groups = is->second;
+      }
     }
   }
   const int hinted_level = had_hint ? level : -1;
@@ -1905,7 +1953,9 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
   RunOutcome ro;
   unsigned int n_groups = 0;
   bool gb_bailed = false, pf_off = false;
+  int attempts = 0;
   for (;;) {
+    attempts++;
     x.check_cancel();
     ScopeTimer t_iter("  agg: lower+alloc+launch+sync");
     pbp = make_pb();
@@ -1988,9 +2038,18 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
     gspec.pf_K = pf_off ? -1 : 0;
     {
       ScopeTimer t_l("    agg: launch_program (incl. sync)");
-      ro = launch_program(x, pb, reg_groups, use_fused ? &fspec : nullptr, true, met, tm.T.n_groups, &n_groups, use_gb ? &gspec : nullptr);
+      ro = launch_program(x, pb, reg_groups, use_fused ? &fspec : nullptr, !speculate, met, tm.T.n_groups, &n_groups, use_gb ? &gspec : nullptr);
     }
     if (met) met->launches += 2;
+    if (speculate) {
+      const RunStatus* hs = ro.deferred;
+      const unsigned int* hg = ro.deferred_extra;
+      x.defer([hs, hg, spec_groups]() {
+        if (hs->overflow || hs->pack_overflow || *hg != spec_groups) throw SpeculationMiss();
+      });
+      n_groups = (unsigned int)spec_groups;
+      break;
+    }
     if (ro.status.pack_overflow && use_gb) {
       gb_bailed = true;  // operands outside the dedicated kernel's ranges: same table size on the general sink
       continue;
@@ -2009,7 +2068,7 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
     }
     level++;
   }
-  {
+  if (!speculate) {
     // remember the smallest table class that holds this many groups (not the level that happened to be used: a small
     // input jumps straight to a table sized for its row count)
     int learnt = level;
@@ -2021,6 +2080,8 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
     x.e->agg_hint[hint_key] = learnt * 4 + pack_mode;
     uint64_t& gh = x.e->agg_groups[hint_key];
     gh = std::max<uint64_t>(gh, n_groups);
+    if (attempts == 1 && n_groups <= SPEC_MAX_GROUPS) x.e->agg_spec[spec_key] = n_groups;
+    else x.e->agg_spec.erase(spec_key);
   }
   PipelineBuilder& pb = *pbp;
   // extraction
@@ -2032,15 +2093,44 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
   if (L.outs.size() > (size_t)VM_MAX_OUT) throw EngineError(B200_ERR_UNSUPPORTED, "too many aggregate output columns");
   A.n_out = (int)L.outs.size();
   A.n_keys = n_keys;
-  DevPtr counter = dev_alloc(16, x.st());
-  CUDA_CHECK(cudaMemsetAsync(counter->ptr, 0, 16, x.st()));
-  A.counter = (unsigned long long*)counter->ptr;
-  A.error = (unsigned int*)((uint8_t*)counter->ptr + 8);
+  // one block for the counter words and every output buffer: cleared as a whole when the group count is speculated, so
+  // that rows the extraction leaves unwritten hold empty values (never stray string pointers) until the task's check
+  const size_t rows = std::max<unsigned int>(n_groups, 1);
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  struct Place { size_t data = 0, valid = 0, aux = 0; };
+  std::vector<Place> place(L.outs.size());
+  size_t blk_bytes = 256;
+  for (size_t j = 0; j < L.outs.size(); j++) {
+    const auto& r = L.outs[j];
+    place[j].data = blk_bytes;
+    blk_bytes += up(rows * phys_width(r.phys));
+    if (r.with_valid) {
+      place[j].valid = blk_bytes;
+      blk_bytes += up(rows);
+    }
+    if (r.kind == AO_KEY_PACKED) {
+      place[j].aux = blk_bytes;
+      blk_bytes += up(rows * 8);
+    }
+  }
+  DevPtr blk = dev_alloc(blk_bytes, x.st());
+  uint8_t* const base = (uint8_t*)blk->ptr;
+  CUDA_CHECK(cudaMemsetAsync(base, 0, speculate ? blk_bytes : 16, x.st()));
+  A.counter = (unsigned long long*)base;
+  A.error = (unsigned int*)(base + 8);
+  A.cap = n_groups;
   uint64_t wbytes = 0;
   for (size_t j = 0; j < L.outs.size(); j++) {
     const auto& r = L.outs[j];
-    DevColumn oc = make_out_column(r.name, r.type, r.phys, n_groups, r.with_valid, x.st());
+    DevColumn oc;
+    oc.name = r.name;
+    oc.type = r.type;
+    oc.phys = r.phys;
     oc.n = n_groups;
+    oc.data = base + place[j].data;
+    if (r.with_valid) oc.valid = base + place[j].valid;
+    oc.nullable = r.with_valid;
+    oc.keep.push_back(blk);
     if (r.key_idx >= 0) {
       for (auto& k : L.keys[(size_t)r.key_idx].keep) oc.keep.push_back(k);
       if (r.phys == PH_STRVIEW) {
@@ -2052,12 +2142,7 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
     AggOut& o = A.out[j];
     o.data = (void*)oc.data;
     o.valid = (uint8_t*)oc.valid;
-    o.aux = nullptr;
-    if (r.kind == AO_KEY_PACKED) {
-      DevPtr ch = dev_alloc((size_t)std::max<unsigned int>(n_groups, 1) * 8, x.st());
-      o.aux = ch->ptr;
-      oc.keep.push_back(ch);
-    }
+    o.aux = r.kind == AO_KEY_PACKED ? base + place[j].aux : nullptr;
     o.kind = r.kind;
     o.a = r.a;
     o.b = r.b;
@@ -2071,7 +2156,7 @@ DevBatchPtr run_aggregate(const Exec& x, const BuilderFactory& make_pb, const Pl
   {
     // the extraction's overflow flag (decimal AVG / SUM precision) only has to be seen before the task returns
     const unsigned int* herr = x.fetch<unsigned int>(A.error);
-    x.defer([herr, counter]() {
+    x.defer([herr, blk]() {
       if (*herr) throw EngineError(B200_ERR_EXECUTION, "Arithmetic overflow");
     });
   }
@@ -2112,6 +2197,28 @@ struct Runner {
         return n_partitions(*n.children[0]);
       case PlanNode::HashJoin: return n_partitions(*n.children[1]);
       default: return n_partitions(*n.children[0]);
+    }
+  }
+
+  // Whether partition 0 of `n` is a single run of rows in the order its producer wrote them: false when a shuffle
+  // reader (possibly under row-preserving operators) concatenates several map outputs, each sorted on its own.
+  bool one_run(const PlanNode& n) {
+    switch (n.op) {
+      case PlanNode::ShuffleReader: {
+        std::lock_guard<std::mutex> g(x.e->mu);
+        auto it = x.e->shuffle.find(ShuffleKey{job, n.reader_stage_id, 0});
+        int pieces = 0;
+        if (it != x.e->shuffle.end())
+          for (auto& p : it->second) pieces += p.r1 > p.r0 ? 1 : 0;
+        return pieces <= 1;
+      }
+      case PlanNode::Passthrough:
+        if (n.op_name == "CoalescePartitionsExec" && n_partitions(*n.children[0]) != 1) return false;
+        return one_run(*n.children[0]);
+      case PlanNode::Filter:
+      case PlanNode::Projection:
+      case PlanNode::Limit: return one_run(*n.children[0]);
+      default: return true;
     }
   }
 
@@ -2332,7 +2439,7 @@ struct Runner {
       case PlanNode::Aggregate: {
         const PlanNode& child = *n.children[0];
         bool all = (n.agg_mode == AggMode::Final || n.agg_mode == AggMode::Single) && part == 0 && n_partitions(child) > 1;
-        out = with_chain(child, part, all, [&](const BuilderFactory& mk, DevBatchPtr& src) { return run_aggregate(x, mk, n, src, met); });
+        out = with_chain(child, part, all, [&](const BuilderFactory& mk, DevBatchPtr& src) { return run_aggregate(x, mk, n, src, met, part); });
         break;
       }
       case PlanNode::HashJoin:
@@ -2345,7 +2452,22 @@ struct Runner {
         break;
       }
       case PlanNode::SortPreservingMerge: {
-        DevBatchPtr in = exec_all(*n.children[0]);
+        const PlanNode& child = *n.children[0];
+        if (n_partitions(child) == 1 && one_run(child)) {
+          // one sorted input: the merge passes it through (DataFusion's SortPreservingMergeExec over one partition)
+          DevBatchPtr in = exec(child, 0);
+          if (met) met->input_rows += (uint64_t)in->n;
+          const int64_t m = n.fetch >= 0 ? std::min<int64_t>(n.fetch, in->n) : in->n;
+          if (m == in->n) {
+            out = in;
+            break;
+          }
+          out = std::make_shared<DevBatch>();
+          out->n = m;
+          for (auto& c : in->cols) out->cols.push_back(slice_column(c, 0, m));
+          break;
+        }
+        DevBatchPtr in = exec_all(child);
         out = do_sort(n.sort_keys, n.fetch, in, met);
         break;
       }
@@ -2484,7 +2606,7 @@ struct Runner {
     proj.n = n;
     for (size_t c = 0; c < n_in_cols; c++) proj.cols.push_back(in->cols[c]);
     DevBatchPtr out = gather_batch(x, proj, (const int64_t*)idx->ptr, m, false);
-    CUDA_CHECK(cudaStreamSynchronize(x.st()));
+    x.wait();
     if (met) {
       met->elapsed_ns += (uint64_t)std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
       met->input_rows += (uint64_t)n;
@@ -2838,6 +2960,12 @@ struct Runner {
   // character bytes of every Utf8 column of `b` (rows [0, b.n)), one read-back for all of them; known values are reused
   std::vector<int64_t> string_bytes(const DevBatch& b) {
     std::vector<int64_t> out;
+    queue_string_bytes(b, out);
+    x.sync();
+    return out;
+  }
+  // the same, with the read-back queued: `out` is complete after the task's next x.sync()
+  void queue_string_bytes(const DevBatch& b, std::vector<int64_t>& out) {
     PartStrCols sc;
     sc.n = 0;
     std::vector<size_t> unknown;
@@ -2864,10 +2992,10 @@ struct Runner {
       CUDA_CHECK(launch_partition_hist(none, b.n, 1, nullptr, (unsigned long long*)acc->ptr, sc, (unsigned long long*)acc->ptr + 1, x.st()));
       x.count();
       const unsigned long long* h = (const unsigned long long*)x.fetch_bytes((const unsigned long long*)acc->ptr + 1, (size_t)sc.n * 8);
-      x.sync();
-      for (size_t k = 0; k < unknown.size(); k++) out[unknown[k]] = (int64_t)h[k];
+      x.defer([h, unknown, &out]() {
+        for (size_t k = 0; k < unknown.size(); k++) out[unknown[k]] = (int64_t)h[k];
+      });
     }
-    return out;
   }
 
   struct FusedExchange {
@@ -3107,8 +3235,8 @@ struct Runner {
       std::vector<int64_t> cb;
       {
         ScopeTimer t2("writer: string bytes + final sync");
-        cb = string_bytes(*st);
-        x.sync();  // deferred status checks of this task's kernels
+        queue_string_bytes(*st, cb);
+        x.sync();  // the string byte counts and the deferred status checks of this task's kernels
       }
       b200_shuffle_write_partition w{};
       w.partition_id = single ? 0u : (uint64_t)input_partition;
@@ -4175,6 +4303,7 @@ void b200_engine_destroy(b200_engine* e) {
   e->tables.clear();
   e->shuffle.clear();
   e->packed_cache.clear();
+  e->plan_cache.clear();
   cudaStreamSynchronize(e->stream);
   for (auto& sl : e->nslot) {
     if (sl.pinned) cudaFreeHost(sl.pinned);
@@ -4212,6 +4341,7 @@ uint64_t b200_engine_counter(b200_engine* e, const char* name) {
   if (n == "groupby") return e->n_groupby;
   if (n == "fastfilter") return e->n_fastfilter;
   if (n == "ingest_bytes_saved") return e->narrowed_bytes_saved;
+  if (n == "stream_syncs") return e->stream_syncs;
   return 0;
 }
 
@@ -4232,6 +4362,7 @@ int b200_engine_set_config(b200_engine* e, const char* key, const char* value) {
     if (std::string(key) == "b200.agg.reset_hints") {
       e->agg_hint.clear();
       e->agg_groups.clear();
+      e->agg_spec.clear();
     }  // forget which aggregate strategy each plan shape needed
     if (std::string(key) == "b200.metrics.kernel_timing") e->kernel_timing = std::string(value) == "on" || std::string(value) == "1" || std::string(value) == "true";
   });
@@ -4457,27 +4588,48 @@ int b200_stage_prepare(b200_engine* e, const char* job_id, int64_t stage_id, con
   ScopeTimer tm("stage_prepare");
   return guard([&] {
     if (!e || !plan_json || !out) throw EngineError(B200_ERR_INVALID, "null argument");
-    Json j = parse_json(plan_json, plan_len ? (size_t)plan_len : strlen(plan_json));
-    PlanPtr plan = parse_plan(j);
-    if (plan->op != PlanNode::ShuffleWriter)
-      throw EngineError(B200_ERR_INVALID, "Plan passed to new_query_stage_exec is not a ShuffleWriterExec");  // execution_engine.rs:164-167
+    const size_t len = plan_len ? (size_t)plan_len : strlen(plan_json);
+    // strategy hints (which aggregate sink / table size worked) are remembered per plan SHAPE: the job id is taken out
+    // of the hashed text so that the next job that runs the same stage plan starts from what the last one learnt
+    std::string shape(plan_json, len);
+    const std::string tag = "\"job_id\":\"";
+    size_t at = shape.find(tag);
+    if (at != std::string::npos) {
+      size_t end = shape.find('"', at + tag.size());
+      if (end != std::string::npos) shape.erase(at + tag.size(), end - at - tag.size());
+    }
+    const std::string stage_tag = std::to_string(stage_id) + ":";
+    // without a job id from the caller the stage takes the plan's own, so the whole text is the key
+    const std::string key = stage_tag + (job_id ? shape : std::string(plan_json, len));
+    std::shared_ptr<const PlanNode> plan;
+    {
+      std::lock_guard<std::mutex> g(e->mu);
+      auto it = e->plan_cache.find(key);
+      if (it != e->plan_cache.end()) {
+        it->second.used = ++e->plan_cache_tick;
+        plan = it->second.plan;
+      }
+    }
+    if (!plan) {
+      PlanPtr parsed = parse_plan(parse_json(plan_json, len));
+      if (parsed->op != PlanNode::ShuffleWriter)
+        throw EngineError(B200_ERR_INVALID, "Plan passed to new_query_stage_exec is not a ShuffleWriterExec");  // execution_engine.rs:164-167
+      parsed->stage_id = stage_id;
+      plan = std::shared_ptr<const PlanNode>(std::move(parsed));
+      std::lock_guard<std::mutex> g(e->mu);
+      if (e->plan_cache.size() >= PLAN_CACHE_ENTRIES) {
+        auto lru = e->plan_cache.begin();
+        for (auto it = e->plan_cache.begin(); it != e->plan_cache.end(); ++it)
+          if (it->second.used < lru->second.used) lru = it;
+        e->plan_cache.erase(lru);
+      }
+      e->plan_cache[key] = b200_engine::CachedPlan{plan, ++e->plan_cache_tick};
+    }
     auto* s = new b200_stage();
     s->eng = e;
     s->job_id = job_id ? job_id : plan->job_id;
     s->stage_id = stage_id;
-    plan->stage_id = stage_id;
-    {
-      // strategy hints (which aggregate sink / table size worked) are remembered per plan SHAPE: the job id is taken out
-      // of the hashed text so that the next job that runs the same stage plan starts from what the last one learnt
-      std::string shape(plan_json, plan_len ? (size_t)plan_len : strlen(plan_json));
-      const std::string tag = "\"job_id\":\"";
-      size_t at = shape.find(tag);
-      if (at != std::string::npos) {
-        size_t end = shape.find('"', at + tag.size());
-        if (end != std::string::npos) shape.erase(at + tag.size(), end - at - tag.size());
-      }
-      s->fingerprint = std::to_string(stage_id) + ":" + std::to_string(mix64(hash_bytes((const uint8_t*)shape.data(), (uint32_t)shape.size())));
-    }
+    s->fingerprint = stage_tag + std::to_string(mix64(hash_bytes((const uint8_t*)shape.data(), (uint32_t)shape.size())));
     collect_nodes(*plan, s);
     s->plan = std::move(plan);
     *out = s;
@@ -4650,30 +4802,41 @@ int b200_stage_execute(b200_stage* s, int input_partition, const volatile int32_
   return guard([&] {
     if (!s || !n_out) throw EngineError(B200_ERR_INVALID, "null argument");
     CUDA_CHECK(cudaSetDevice(s->eng->device));
-    Exec x{s->eng, s, cancel_flag};
-    Runner r{x, s->job_id};
     std::vector<b200_shuffle_write_partition> res;
-    try {
-      res = r.execute_stage(*s->plan, input_partition);
-    } catch (...) {
+    // a cancelled or failed task leaves nothing behind (Executor::cancel_task drops the future together with
+    // its partial outputs, executor.rs:217-237): remove whatever this task already stored
+    auto discard = [&]() {
+      s->eng->stream_syncs++;
       cudaStreamSynchronize(s->eng->stream);
       Exec::abandon();
-      // a cancelled or failed task leaves nothing behind (Executor::cancel_task drops the future together with
-      // its partial outputs, executor.rs:217-237): remove whatever this task already stored
-      {
-        std::lock_guard<std::mutex> g(s->eng->mu);
-        for (auto it = s->eng->shuffle.begin(); it != s->eng->shuffle.end();) {
-          if (it->first.job == s->job_id && it->first.stage == s->stage_id) {
-            auto& v = it->second;
-            v.erase(std::remove_if(v.begin(), v.end(), [&](const Piece& pc) { return (pc.file_id == input_partition || (pc.file_id < 0 && it->first.part == input_partition)) && pc.src_rank == s->eng->rank; }), v.end());
-            if (v.empty()) {
-              it = s->eng->shuffle.erase(it);
-              continue;
-            }
+      std::lock_guard<std::mutex> g(s->eng->mu);
+      for (auto it = s->eng->shuffle.begin(); it != s->eng->shuffle.end();) {
+        if (it->first.job == s->job_id && it->first.stage == s->stage_id) {
+          auto& v = it->second;
+          v.erase(std::remove_if(v.begin(), v.end(), [&](const Piece& pc) { return (pc.file_id == input_partition || (pc.file_id < 0 && it->first.part == input_partition)) && pc.src_rank == s->eng->rank; }), v.end());
+          if (v.empty()) {
+            it = s->eng->shuffle.erase(it);
+            continue;
           }
-          ++it;
         }
+        ++it;
       }
+    };
+    const std::vector<OpMetrics> metrics0 = s->metrics;
+    try {
+      try {
+        Runner r{Exec{s->eng, s, cancel_flag, true}, s->job_id};
+        res = r.execute_stage(*s->plan, input_partition);
+      } catch (const SpeculationMiss&) {
+        // an aggregate's groups differed from the last run of its shape: the writers store only after the task's final
+        // synchronisation, so nothing of the first run is visible; run the task once more without guessing
+        discard();
+        s->metrics = metrics0;
+        Runner r{Exec{s->eng, s, cancel_flag, false}, s->job_id};
+        res = r.execute_stage(*s->plan, input_partition);
+      }
+    } catch (...) {
+      discard();
       throw;
     }
     if ((int)res.size() > cap) throw EngineError(B200_ERR_INVALID, "output array too small");
@@ -4707,6 +4870,7 @@ int b200_stage_execute_exchange(b200_stage* s, int input_partition, const volati
         ex.run(&sent, &recvd);
       }
     } catch (...) {
+      e->stream_syncs++;
       cudaStreamSynchronize(e->stream);
       Exec::abandon();
       throw;

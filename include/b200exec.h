@@ -77,7 +77,8 @@ uint64_t b200_engine_kernel_launches(b200_engine* e);
 /* Introspection for tests and bench.py: how many pipelines ran on which kernel family so far.
  * name: "fused" (fused.cuh kernel, any variant), "fused_static" (an ahead-of-time shape),
  * "vm" (tile VM pipeline_kernel); "ingest_bytes_saved": host->device bytes NOT sent because
- * Decimal128 values were narrowed on the host and widened on the device.  Unknown names return 0. */
+ * Decimal128 values were narrowed on the host and widened on the device; "stream_syncs": host waits on the
+ * engine's stream inside stage tasks and partition exports.  Unknown names return 0. */
 uint64_t b200_engine_counter(b200_engine* e, const char* name);
 /* Per-kernel-family device time (CUDA events on the launching stream) and algorithmic bytes, accumulated since the
  * last reset while the config key "b200.metrics.kernel_timing" is "on" (radix partition, join build / probe,
